@@ -2,10 +2,15 @@
 """Benchmark of the hot path named by BASELINE.json: differentiable env-steps/s (forward + adjoint).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-cuda] [--env AntEnv] [--num-envs 4096]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one short-horizon rollout of the workload: ``horizon`` env-steps forward for ``num_envs`` environments
-per GPU, then the adjoint of all of them.  Headline workload = BASELINE.json configs[1]: AntEnv, 4096 envs, SHAC
+per GPU, then the adjoint of all of them.  Every timed loop (kernel path, end-to-end graphed and eager, each config) runs
+K steps.  ``--dump-outputs DIR`` writes what the last timed step of the headline workload computed, as float32
+``DIR/<name>.npy``: ``kernel_*`` (final q / qd, gradients w.r.t. the initial state and every step's joint_act) and
+``e2e_loss`` / ``e2e_grad_actions`` (what the graphed rollout hands back); inputs are seeded, so two builds can be
+compared output for output.  Headline workload = BASELINE.json configs[1]: AntEnv, 4096 envs, SHAC
 horizon 32 (SURVEY.md section 8d).  Prints ONE JSON line (rank 0):
 
 * ``e2e``      THE HEADLINE: env-steps/s through the reference-facing API -- ``envs.<Env>.step`` (action map, ``dflex.sim.
@@ -245,11 +250,31 @@ def run_reference_cuda(args):
 
 
 # ------------------------------------------------------------------------------------------------ our arm
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, num_envs):
+    """Write ``arrays`` (name -> (tensor, axis of the environments or None)) as ``out_dir/<name>.npy`` in float32.  When they
+    exceed DUMP_BYTES together, every array keeps the same fixed, seeded sample of environments (in index order)."""
+    import numpy as np
+    total = sum(t.numel() * 4 for t, _ in arrays.values())
+    keep = None
+    if total > DUMP_BYTES:
+        k = max(1, num_envs * DUMP_BYTES // total)
+        keep = np.sort(np.random.default_rng(0).choice(num_envs, k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (t, axis) in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if keep is not None and axis is not None:
+            a = np.take(a, keep, axis=axis)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32, copy=False))
+
+
 def measure_config(env_name, N, T, steps, warmup, dev, rank, world, dist, e2e_mode="graph", comm_floats=0,
-                   ncu_range=False, ncu_range_e2e=False, clocks=None, tape_dtype="fp32"):
+                   ncu_range=False, ncu_range_e2e=False, clocks=None, tape_dtype="fp32", dump_dir=None):
     """Kernel path + end-to-end numbers of one workload on this rank.  Returns a dict of raw timings and geometry.
     tape_dtype "bf16": the adjoint tape stores (v, a, f_tot) of every row as bf16 (BASELINE config C2 "bf16 states"; arithmetic
-    and the state stay fp32)."""
+    and the state stay fp32).  dump_dir: write what the last timed step of each path computed there (``dump_outputs``)."""
     import torch
     import diffrl_b200
     from diffrl_b200 import _capi
@@ -301,13 +326,13 @@ def measure_config(env_name, N, T, steps, warmup, dev, rank, world, dist, e2e_mo
             tapes.append(tape)
         if record:
             ev3[1].record()
-        gq, gqd = gq_seed, gqd_seed
+        gq, gqd, gacts, gms = gq_seed, gqd_seed, [None] * T, [None] * T
         for t in reversed(range(T)):
-            gq, gqd, gact, gm = eng.backward(acts[t], muscs[t], tapes[t], gq, gqd, S, mm, dt)
+            gq, gqd, gacts[t], gms[t] = eng.backward(acts[t], muscs[t], tapes[t], gq, gqd, S, mm, dt)
         if record:
             ev3[2].record()
             phase_events.append(ev3)
-        return gq
+        return q, qd, gq, gqd, gacts, gms      # what a caller of this path receives
 
     for _ in range(warmup):
         kernel_rollout()
@@ -321,7 +346,7 @@ def measure_config(env_name, N, T, steps, warmup, dev, rank, world, dist, e2e_mo
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
     ev[0].record()
     for _ in range(steps):
-        kernel_rollout(record=True)
+        kernel_out = kernel_rollout(record=True)
     ev[1].record()
     barrier()
     kernel_ms = ev[0].elapsed_time(ev[1])
@@ -363,7 +388,7 @@ def measure_config(env_name, N, T, steps, warmup, dev, rank, world, dist, e2e_mo
         torch.cuda.current_stream().synchronize()
         return float(host_loss)
 
-    e2e_steps = max(1, steps // 2)
+    e2e_steps = steps
     for _ in range(max(1, warmup // 2)):
         e2e_rollout()
     barrier()
@@ -374,6 +399,7 @@ def measure_config(env_name, N, T, steps, warmup, dev, rank, world, dist, e2e_mo
     e3[1].record()
     barrier()
     eager_ms = e3[0].elapsed_time(e3[1])
+    e2e_out = (host_loss, host_grad)
 
     # the same rollout through the package's graphed-rollout API (one CUDA graph per rollout: H2D actions,
     # horizon x env.step, loss.backward, D2H loss + action gradients)
@@ -407,7 +433,18 @@ def measure_config(env_name, N, T, steps, warmup, dev, rank, world, dist, e2e_mo
         barrier()
         e2e_ms = e3[0].elapsed_time(e3[1])
         e2e_api = "diffrl_b200.rollout.GraphedRollout(envs.%s): one CUDA graph = H2D actions + %d x env.step + backward + D2H" % (env_name, T)
+        e2e_out = (roll.host_loss.clone(), roll.host_grad.clone())
         del roll
+
+    if dump_dir:
+        q, qd, gq, gqd, gacts, gms = kernel_out
+        arrays = {"kernel_q": (q.view(N, Q), 0), "kernel_qd": (qd.view(N, D), 0), "kernel_grad_q0": (gq.view(N, Q), 0),
+                  "kernel_grad_qd0": (gqd.view(N, D), 0), "kernel_grad_joint_act": (torch.stack(gacts).view(T, N, D), 1),
+                  "e2e_loss": (e2e_out[0], None), "e2e_grad_actions": (e2e_out[1], 1)}
+        if M:
+            arrays["kernel_grad_muscle_act"] = (torch.stack(gms).view(T, N, M), 1)
+        dump_outputs(dump_dir, arrays, N)
+    del kernel_out, e2e_out
 
     tile = int(lib.dfx_pack_query(eng.pack, 9))
     row = int(lib.dfx_pack_query(eng.pack, 8))   # DFX_QUERY_TAPE_ROW_FLOATS
@@ -503,16 +540,17 @@ def run_ours(args):
     comm_floats = 16384     # the Ant actor's flattened gradient (cfg/shac/ant.yaml); one all-reduce per rollout when world > 1
     with ClockSampler(local) as clocks:
         head = measure_config(env_name, N, T, args.steps, args.warmup, dev, rank, world, dist, e2e_mode=args.e2e,
-                              comm_floats=comm_floats, ncu_range=args.ncu_range, ncu_range_e2e=args.ncu_range_e2e)
+                              comm_floats=comm_floats, ncu_range=args.ncu_range, ncu_range_e2e=args.ncu_range_e2e,
+                              dump_dir=args.dump_outputs if rank == 0 else None)
     # ---- the other named configs (BASELINE.json): short runs, same measurement
     subs = {}
     if not args.no_configs:
         plan = []
         if world > 1:
-            plan.append(("c4", "AntEnv", 8192, 32, max(2, args.steps // 2), 2))
+            plan.append(("c4", "AntEnv", 8192, 32, args.steps, 2))
         else:
-            plan += [("humanoid8192", "HumanoidEnv", 8192, 32, 2, 1), ("humanoid8192_bf16_tape", "HumanoidEnv", 8192, 32, 2, 1),
-                     ("snu4096_bptt128", "SNUHumanoidEnv", 4096, 128, 2, 1), ("cartpole64", "CartPoleSwingUpEnv", 64, 32, 4, 2)]
+            plan += [("humanoid8192", "HumanoidEnv", 8192, 32, args.steps, 1), ("humanoid8192_bf16_tape", "HumanoidEnv", 8192, 32, args.steps, 1),
+                     ("snu4096_bptt128", "SNUHumanoidEnv", 4096, 128, args.steps, 1), ("cartpole64", "CartPoleSwingUpEnv", 64, 32, args.steps, 2)]
         for key, e, n, t, k, w in plan:
             try:
                 subs[key] = measure_config(e, n, t, k, w, dev, rank, world, dist, e2e_mode=args.e2e, comm_floats=comm_floats,
@@ -589,6 +627,9 @@ def main():
     ap.add_argument("--cpu-procs", type=int, default=0, help="reference arm: host processes (default: one per core of the affinity mask)")
     ap.add_argument("--ncu-range-e2e", action="store_true",
                     help="wrap one graphed end-to-end rollout in cudaProfilerStart/Stop (for ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step of the headline workload computed as DIR/<name>.npy "
+                         "(float32; inputs are seeded, so two builds can be compared output for output)")
     ap.add_argument("--ncu-range", action="store_true",
                     help="wrap ONE kernel-path step in cudaProfilerStart/Stop (use with ncu --profile-from-start off)")
     args = ap.parse_args()

@@ -111,26 +111,26 @@ def test_cuda_matches_oracles_at_named_size(name, N):
 
 def test_snu_bptt128_rollout_matches_reference_kernels():
     """C3's shape: a 128-env-step BPTT window of the muscle humanoid on 4 environments, the GPU kernels against the
-    reference's OWN generated CPU kernels (oracle/_ref/kernels.so through oracle/ref_driver.py).  Forward: every env-step
-    from the reference's state (the chaotic dynamics would amplify a 1e-7 rounding difference over 6144 substeps; the
-    per-step comparison is the one that can hold 1e-5-class tolerances), plus the free-running GPU trajectory for the
-    first steps.  Adjoint: the full 128-step chain of cotangents through both implementations' tapes."""
+    reference's OWN generated CPU kernels (their results recorded in tests/golden/ref_kernels.npz by
+    oracle/make_ref_kernel_golden.py).  Forward: every env-step from the reference's state (the chaotic dynamics would
+    amplify a 1e-7 rounding difference over 6144 substeps; the per-step comparison is the one that can hold 1e-5-class
+    tolerances), plus the free-running GPU trajectory for the first steps.  Adjoint: the full 128-step chain of cotangents
+    through both implementations' tapes."""
     import torch
-    import ref_driver
-    if not ref_driver.available():
-        pytest.skip("oracle/_ref/kernels.so not built (build container: python oracle/make_golden.py)")
+    import make_ref_kernel_golden as rkg
     from diffrl_b200.engine import ArticulationEngine
     from diffrl_b200.modelpack import articulation_from_model
-    name, n, T = "SNUHumanoidEnv", 4, 128
+    name, n, T = "SNUHumanoidEnv", rkg.SNU_ENVS, rkg.SNU_STEPS
     d, model = load_golden(name)
-    arrays = dict(np.load(os.path.join(ROOT, "diffrl_b200", "assets", name + ".npz")))
+    gold = np.load(os.path.join(ROOT, "tests", "golden", "ref_kernels.npz"))
+    ref = {k[len("snu_bptt128/"):]: torch.from_numpy(gold[k]) for k in gold.files if k.startswith("snu_bptt128/")}
     S, mm, dt = int(d["meta/substeps"]), int(d["meta/mass_matrix_freq"]), float(d["meta/dt"])
-    rm = ref_driver.RefModel(arrays, n, ground=True)
     desc, _ = articulation_from_model(model, int(d["meta/num_envs"]))
     eng = ArticulationEngine(desc, n, "cuda:0")
     Q, D, M = desc.Q, desc.D, desc.M
-    g = torch.Generator().manual_seed(5)
-    q, qd = rm.m.joint_q.clone(), rm.m.joint_qd.clone()
+    assert ref["q"].shape == (T + 1, n * Q) and ref["qd"].shape == (T + 1, n * D)
+    g = torch.Generator().manual_seed(rkg.SNU_SEED)
+    q, qd = ref["q"][0], ref["qd"][0]
     act = torch.zeros(n * D)
     cu = lambda x: x.to("cuda:0").contiguous()
     ref_states, muscs, tapes_gpu = [], [], []
@@ -138,8 +138,10 @@ def test_snu_bptt128_rollout_matches_reference_kernels():
     tol = fwd_rtol(name)
     free_err = []
     for t in range(T):
-        musc = torch.rand(n * M, generator=g) * 40.0          # activation x strength range of the env (envs/snu_humanoid.py:283-296)
-        q_ref, qd_ref, _, _ = ref_driver.env_step(rm, q, qd, act, musc, dt, S, mm)
+        musc = rkg.snu_musc(g, n * M)
+        if t == 0:        # the recorded run drew the same activations
+            assert torch.equal(musc[: ref["musc_head"].numel()], ref["musc_head"])
+        q_ref, qd_ref = ref["q"][t + 1], ref["qd"][t + 1]
         gq_, gqd_, tape, _ = eng.forward(cu(q), cu(qd), cu(act), cu(musc), S, mm, dt)        # from the REFERENCE's state
         err = max(float((gq_.cpu() - q_ref).abs().max() / q_ref.abs().max()), float((gqd_.cpu() - qd_ref).abs().max() / (qd_ref.abs().max() + 1.0)))
         worst_step = max(worst_step, err)
@@ -153,47 +155,43 @@ def test_snu_bptt128_rollout_matches_reference_kernels():
     # adjoint chain over the whole window (cotangent 1 on the final state): the reference's cotangents are propagated, the GPU
     # adjoint of every env-step gets the reference's incoming cotangents (per-step adjoint parity; the chain's own
     # conditioning would otherwise dominate after a few steps)
-    gq_r, gqd_r = torch.ones(n * Q), torch.ones(n * D)
-    rows, cots = [], {}
-    for t in reversed(range(T)):
+    # (the recorded chain stops where the reference's own cotangents overflowed fp32: nothing left to compare beyond)
+    rows, cots, gm_errs = [], {}, []
+    for k in range(ref["ref_jump"].shape[0]):
+        t = T - 1 - k
+        gq_r, gqd_r = ref["cot_q"][k], ref["cot_qd"][k]
         cots[t] = (gq_r, gqd_r)
-        q0, qd0 = ref_states[t]
-        _, _, grads, _ = ref_driver.env_step(rm, q0, qd0, act, muscs[t], dt, S, mm, gq_out=gq_r, gqd_out=gqd_r)
-        gq_n, gqd_n, _, gm_r = grads
+        gq_n, gqd_n = ref["cot_q"][k + 1], ref["cot_qd"][k + 1]
         gq_g, gqd_g, _, gm_g = eng.backward(cu(act), cu(muscs[t]), tapes_gpu[t], cu(gq_r), cu(gqd_r), S, mm, dt)
         scale = float(max(gq_n.abs().max(), gqd_n.abs().max()))
-        if not np.isfinite(scale) or scale > 1e12:
-            break                                   # the reference's own cotangents overflowed fp32: nothing left to compare
+        e_gm = 0.0
+        if k % rkg.GRAD_MUSC_EVERY == 0:            # the recorded sample of the muscle-activation gradients
+            gm_r = ref["grad_musc"][k // rkg.GRAD_MUSC_EVERY]
+            e_gm = float((gm_g.cpu() - gm_r).abs().max() / (gm_r.abs().max() + 1e-30))
+            gm_errs.append(e_gm)
         rows.append((t, float((gq_g.cpu() - gq_n).abs().max()) / scale, float((gqd_g.cpu() - gqd_n).abs().max()) / scale,
-                     float((gm_g.cpu() - gm_r).abs().max() / (gm_r.abs().max() + 1e-30)), scale))
-        gq_r, gqd_r = gq_n, gqd_n
+                     e_gm, scale, float(ref["ref_jump"][k])))
     assert len(rows) >= 64, len(rows)
-    for col, what in ((1, "gq"), (2, "gqd"), (3, "gmusc")):
-        errs = np.array([r[col] for r in rows])
+    for errs, what in (([r[1] for r in rows], "gq"), ([r[2] for r in rows], "gqd"), (gm_errs, "gmusc")):
+        errs = np.array(errs)
         assert np.median(errs) < GRAD_RTOL and np.quantile(errs, 0.9) < 4 * GRAD_RTOL, (what, float(np.median(errs)), float(np.quantile(errs, 0.9)))
     # a step outside 8 x the tolerance must sit on a switching surface of the contact / limit model: the reference's (or the
     # kernels') own gradient of that step jumps by a comparable amount when the step's input state moves by 1-4 fp32 ulp
     outliers = [r for r in rows if max(r[1:4]) >= 8 * GRAD_RTOL]
     assert len(outliers) <= max(2, len(rows) // 20), [(r[0], max(r[1:4])) for r in outliers]
-    rng = np.random.default_rng(11)
     for r in outliers:
         t = r[0]
         q0, qd0 = ref_states[t]
         cot = cots[t]
-        base = ref_driver.env_step(rm, q0, qd0, act, muscs[t], dt, S, mm, gq_out=cot[0], gqd_out=cot[1])[2]
         _, _, tape0, _ = eng.forward(cu(q0), cu(qd0), cu(act), cu(muscs[t]), S, mm, dt)
         gbase = eng.backward(cu(act), cu(muscs[t]), tape0, cu(cot[0]), cu(cot[1]), S, mm, dt)
-        jump = 0.0
-        for mag in (1.2e-7, 4.8e-7):                 # random sign patterns of 1 and 4 ulp: a switching surface nearby flips for some
-            for _ in range(6):
-                sq = torch.tensor(rng.choice([-1.0, 1.0], q0.numel()), dtype=torch.float32)
-                sqd = torch.tensor(rng.choice([-1.0, 1.0], qd0.numel()), dtype=torch.float32)
-                qp, qdp = q0 * (1.0 + mag * sq), qd0 * (1.0 + mag * sqd)
-                pert = ref_driver.env_step(rm, qp, qdp, act, muscs[t], dt, S, mm, gq_out=cot[0], gqd_out=cot[1])[2]
-                _, _, tp, _ = eng.forward(cu(qp), cu(qdp), cu(act), cu(muscs[t]), S, mm, dt)
-                gp = eng.backward(cu(act), cu(muscs[t]), tp, cu(cot[0]), cu(cot[1]), S, mm, dt)
-                jump = max(jump, float((pert[0] - base[0]).abs().max()) / r[4], float((pert[1] - base[1]).abs().max()) / r[4],
-                           float((gp[0] - gbase[0]).abs().max()) / r[4], float((gp[1] - gbase[1]).abs().max()) / r[4])
+        jump = r[5]                                  # the reference's own jump under the same perturbations (recorded)
+        # random sign patterns of 1 and 4 ulp: a switching surface nearby flips for some
+        for fq, fqd in rkg.perturbations(t, q0.numel(), qd0.numel()):
+            qp, qdp = q0 * fq, qd0 * fqd
+            _, _, tp, _ = eng.forward(cu(qp), cu(qdp), cu(act), cu(muscs[t]), S, mm, dt)
+            gp = eng.backward(cu(act), cu(muscs[t]), tp, cu(cot[0]), cu(cot[1]), S, mm, dt)
+            jump = max(jump, float((gp[0] - gbase[0]).abs().max()) / r[4], float((gp[1] - gbase[1]).abs().max()) / r[4])
         assert max(r[1:4]) <= 8.0 * jump, ("step %d: adjoint error %.2e, largest jump of the reference's / the kernels' own gradient "
                                            "under 1-4 ulp input perturbations %.2e" % (t, max(r[1:4]), jump))
 

@@ -2,7 +2,8 @@
 * fp32 forward  == golden trajectories recorded from the unmodified reference, BIT FOR BIT;
 * fp64 central finite differences of the oracle == the reference's reverse-mode gradients
   (an adjoint-free confirmation of what the hand-derived CUDA adjoint must reproduce);
-* fp32 forward  == the reference's own compiled kernels (oracle/_ref) on fresh random states, bit for bit."""
+* fp32 forward  == the reference's own compiled kernels on fresh random states, bit for bit (their results recorded
+  in tests/golden/ref_kernels.npz by oracle/make_ref_kernel_golden.py)."""
 import os
 import sys
 
@@ -69,22 +70,11 @@ def test_finite_difference_gradient_matches_reference_adjoint(name):
 
 @pytest.mark.parametrize("name", ["AntEnv", "SNUHumanoidEnv", "CartPoleSwingUpEnv"])
 def test_oracle_equals_reference_kernels_on_random_states(name):
-    import ref_driver
-    if not ref_driver.available():
-        pytest.skip("oracle/_ref/kernels.so not built (build container only)")
-    import torch
+    """Inputs and the reference kernels' results: tests/golden/ref_kernels.npz (oracle/make_ref_kernel_golden.py)."""
     d, model, o, c = _setup(name)
-    N, Q, D, M = 5, o.desc.Q, o.desc.D, o.desc.M
-    rng = np.random.default_rng(11)
-    p = "case%d/" % (int(d["meta/num_cases"]) - 1)
-    pick = rng.integers(0, c["N"], N)
-    q0 = (d[p + "q0"].reshape(c["N"], Q)[pick] + 1e-2 * rng.standard_normal((N, Q))).astype(np.float32)
-    qd0 = (d[p + "qd0"].reshape(c["N"], D)[pick] + 1e-1 * rng.standard_normal((N, D))).astype(np.float32)
-    act = (d[p + "act"].reshape(c["N"], D)[pick] * rng.uniform(0.5, 1.5, (N, D))).astype(np.float32)
-    musc = (d[p + "musc"].reshape(c["N"], M)[pick] * rng.uniform(0.5, 1.5, (N, M))).astype(np.float32) if M else None
-    arrays = dict(np.load(os.path.join(ROOT, "diffrl_b200", "assets", name + ".npz")))
-    rm = ref_driver.RefModel(arrays, N, ground=bool(d["meta/ground"]))
-    t = lambda a: None if a is None else torch.tensor(a.ravel())
-    rq, rqd, _, _ = ref_driver.env_step(rm, t(q0), t(qd0), t(act), t(musc), c["dt"], c["S"], c["mm"])
-    oq, oqd = o.forward(q0, qd0, act, musc, c["S"], c["mm"], c["dt"])
-    assert np.array_equal(oq.astype(np.float32), rq.numpy()) and np.array_equal(oqd.astype(np.float32), rqd.numpy())
+    g = np.load(os.path.join(ROOT, "tests", "golden", "ref_kernels.npz"))
+    p = "random/%s/" % name
+    musc = g[p + "musc"] if (p + "musc") in g.files else None
+    assert g[p + "q0"].shape[0] == 5 and (musc is None) == (o.desc.M == 0)
+    oq, oqd = o.forward(g[p + "q0"], g[p + "qd0"], g[p + "act"], musc, c["S"], c["mm"], c["dt"])
+    assert np.array_equal(oq.astype(np.float32), g[p + "q"]) and np.array_equal(oqd.astype(np.float32), g[p + "qd"])
